@@ -280,7 +280,7 @@ def run_ours(args):
     # ================= headline: replicas (N=1: the single window) =================
     full_inputs = synth_inputs(F, wl["n_cond"], h, w, seed=rank)
     host = {k: (v.to(torch.bfloat16) if v.dtype.is_floating_point else v).pin_memory() for k, v in full_inputs.items()}
-    step_resident, lat_res, _ = make_stepper(pipe, full_inputs, wl["domain"])
+    step_resident, lat_res, ts_res = make_stepper(pipe, full_inputs, wl["domain"])
 
     out_host = torch.empty_like(host["latents"]).pin_memory()
     ts_host = torch.empty_like(host["ts"]).pin_memory()
@@ -320,6 +320,11 @@ def run_ours(args):
     sampler.start()
     ms_res = timed(step_resident, args.steps, max(args.warmup, 3))
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # what denoise_window hands back to its caller after the last timed step: the window's latents and timestep
+        # indices, both updated in place
+        dump_outputs(args.dump_outputs, {"latents": lat_res.float().cpu().numpy(),
+                                         "timestep_indices": ts_res.cpu().double().numpy()})
     ms_e2e = timed(step_e2e, args.steps, 1)
     assert torch.isfinite(out_host.float()).all(), "non-finite latents out of the window step"
 
@@ -447,6 +452,15 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes every array as ``out_dir/<name>.npy``, so two builds run with the same arguments (hence the same seeded
+    inputs and weights) can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def gpu_eager_baseline(cfg, sd, inputs, dev, steps):
     """The same window step as the reference would execute it on THIS GPU: the oracle's torch graph in bf16 on
     cuDNN / cuBLAS / SDPA (eager).  A reported comparator like cpu_baseline -- never part of the product path."""
@@ -500,7 +514,11 @@ def main():
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true", help="N>1: skip the frame-sharded `sharded` object")
     ap.add_argument("--quick", action="store_true", help="N=1: headline only (no `also`, no baselines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the latents and timestep indices "
+                    "of the last headline step (rank 0's window) as DIR/<name>.npy in float32 / float64")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

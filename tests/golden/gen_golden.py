@@ -1,5 +1,5 @@
-"""Generate golden fixtures by RUNNING code from /root/reference (only possible in the build
-container -- /root/reference does not exist on the GPU box, so the outputs are committed).
+"""Generate golden fixtures by RUNNING code from a checkout of the original Diffuman4D repository (zju3dv/Diffuman4D).
+The outputs are committed, so the tests never need that checkout.
 
 Pinned here:
   pose_encoder.pt   -- the reference ``PoseEncoder`` (src/diffusers/models/unets/pose_encoder.py), imported
@@ -26,7 +26,11 @@ Pinned here:
                        Weights come from ``diffuman4d_b200.weights.random_state_dict`` loaded with strict=True, which
                        also pins the product's diffusers-layout key/shape spec against the reference module tree.
 
-Run:  python tests/golden/gen_golden.py      (from the repo root, inside the build container)
+Every fixture stays under 1 MB: the pixel-resolution skeletons are drawn as float16-representable values and stored as
+float16 (exact; the tests upcast them to float32), and pipeline_ref.pt keeps only the latent-resolution inputs the tests
+feed to the oracle, not the pixel-resolution images and masks the reference encoded them from.
+
+Run:  python tests/golden/gen_golden.py <Diffuman4D checkout>      (from the repo root)
 """
 import importlib.util
 import os
@@ -36,7 +40,7 @@ import types
 import torch
 import torch.nn as nn
 
-REF = "/root/reference"
+REF = None  # the Diffuman4D checkout, set from the command line
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 
@@ -433,10 +437,11 @@ def gen_unet():
             B = nf * len(domains)
             x = torch.randn(B, cfg.in_channels, h, w, generator=g)
             t = torch.randint(0, 1000, (B,), generator=g)
-            sk = (torch.rand(B, 3, 8 * h, 8 * w, generator=g) * 2 - 1) if cfg.enable_pose_encoder else None
+            sk = (torch.rand(B, 3, 8 * h, 8 * w, generator=g) * 2 - 1).half().float() if cfg.enable_pose_encoder else None
             with torch.no_grad():
                 y = model(x, t, skeletons=sk, domains=domains, num_frames=nf, return_dict=False)[0]
-            runs[dom_tag] = {"sample": x, "timestep": t, "skeletons": sk, "domains": domains, "num_frames": nf, "out": y}
+            runs[dom_tag] = {"sample": x, "timestep": t, "skeletons": None if sk is None else sk.half(), "domains": domains,
+                             "num_frames": nf, "out": y}
             print("unet", tag, dom_tag, tuple(y.shape), float(y.abs().mean()))
         out["cases"][tag] = {"cfg": cfg.to_dict(), "seed": 5, "ref_state_dict_shapes": ref_keys, "runs": runs}
     # the reference's own argument check (UNET:524-525)
@@ -591,7 +596,8 @@ def gen_pipeline():
         mask = torch.ones(F_, 1, h, w)
         mask[:2] = 0
         inp = {"latents": rn(F_, 4, h, w), "pixel_latents": rn(F_, 4, h, w), "plucker": rn(F_, 6, h, w).clamp(-1, 1),
-               "skeletons": (torch.rand(F_, 3, 8 * h, 8 * w, generator=g) * 2 - 1) if pose else rn(F_, 4, h, w),
+               "skeletons": ((torch.rand(F_, 3, 8 * h, 8 * w, generator=g) * 2 - 1) if pose
+                             else rn(F_, 4, h, w)).half().float(),
                "cond_mask": mask, "timestep_indices": torch.tensor([0, 0, 1, 2, 3])}
         schedulers, timesteps = pipe.parepare_schedulers(6, F_)
         ti = inp["timestep_indices"].clone()
@@ -599,7 +605,8 @@ def gen_pipeline():
                    skeletons_latents=inp["skeletons"].clone(), cond_masks_latents=inp["cond_mask"].clone(),
                    latents=inp["latents"].clone(), domains=["spatial"], num_inference_steps=2, schedulers=schedulers,
                    timesteps=timesteps, timestep_indices=ti, guidance_scale=guidance, output_type="latent")
-        out["cases"][tag] = {"pose": pose, "guidance": guidance, "prediction_type": pred, "n_steps_table": 6, "in": inp,
+        out["cases"][tag] = {"pose": pose, "guidance": guidance, "prediction_type": pred, "n_steps_table": 6,
+                             "in": {**inp, "skeletons": inp["skeletons"].half()},
                              "timesteps_table": timesteps.clone(), "out_latents": res, "out_timestep_indices": ti}
         print("pipeline", tag, float(res.abs().mean()), ti.tolist())
 
@@ -623,7 +630,7 @@ def gen_pipeline():
         mask[:n_in] = 0
         pixel = torch.rand(n, 3, 8 * h, 8 * w, generator=g) * 2 - 1
         inp = {"pixel_values": pixel, "plucker": rn(n, 6, h, w).clamp(-1, 1),
-               "skeletons": torch.rand(n, 3, 8 * h, 8 * w, generator=g) * 2 - 1, "cond_masks": mask,
+               "skeletons": (torch.rand(n, 3, 8 * h, 8 * w, generator=g) * 2 - 1).half().float(), "cond_masks": mask,
                "latents": rn(n, 4, h, w), "timestep_indices": torch.zeros(n, dtype=torch.int64)}
         inp["plucker"][:, 0, 0, 0] = torch.arange(n, dtype=torch.float32) / 100
         res = pipe.sliding_iterative_denoise(
@@ -634,8 +641,10 @@ def gen_pipeline():
         z = torch.nn.functional.avg_pool2d(pixel, 8)
         inp["pixel_latents"] = torch.cat([z, z.mean(dim=1, keepdim=True)], dim=1)  # what the fake VAE encoded
         inp["cond_mask_latents"] = torch.nn.functional.interpolate(mask, size=(h, w), mode="nearest")
+        stored = {k: v for k, v in inp.items() if k not in ("pixel_values", "cond_masks")}
+        stored["skeletons"] = inp["skeletons"].half()
         out["cases"][tag] = {"domain": domain, "window_size": ws, "sliding_stride": stride, "bidirectional": bidir,
-                             "alternation_rounds": rounds, "in": inp, "out_latents": res["latents"],
+                             "alternation_rounds": rounds, "in": stored, "out_latents": res["latents"],
                              "out_timestep_indices": res["timestep_indices"], "fully_denoised": res["fully_denoised"],
                              "window_timestep_indices": [w_["timestep_indices"] for w_ in windows],
                              "window_frames": [w_["frames"] for w_ in windows], "n_input": n_in}
@@ -737,6 +746,9 @@ def gen_sampler():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "src", "diffusers")):
+        raise SystemExit("usage: python tests/golden/gen_golden.py <Diffuman4D checkout>")
+    REF = os.path.abspath(sys.argv[1])
     gen_sampler()
     gen_unet()
     gen_pipeline()

@@ -1,4 +1,4 @@
-"""CPU tests: the oracle against the golden vectors produced by code run from /root/reference
+"""CPU tests: the oracle against the golden vectors produced by code run from the original Diffuman4D repository
 (tests/golden/gen_golden.py), and the oracle's own invariants (the reference's runtime checks, SURVEY.md section 4)."""
 import os
 
@@ -130,8 +130,9 @@ def test_oracle_unet_matches_reference_unet_golden(tag):
     m.load_state_dict(random_state_dict(cfg, seed=c["seed"], dtype=torch.float32), strict=True)
     m.eval()
     for r in c["runs"].values():
+        sk = None if r["skeletons"] is None else r["skeletons"].float()   # stored as float16, exactly
         with torch.no_grad():
-            y = m(r["sample"], r["timestep"], r["skeletons"], r["domains"], r["num_frames"])
+            y = m(r["sample"], r["timestep"], sk, r["domains"], r["num_frames"])
         torch.testing.assert_close(y, r["out"], rtol=2e-4, atol=2e-5)
 
 
@@ -166,7 +167,7 @@ def test_window_step_matches_reference_pipeline_golden(tag):
     cin = 4 + 6 + (0 if c["pose"] else 4) + 1
     lat, ti = denoise_window_oracle(
         _fake_unet(cin), s, latents=i["latents"].clone(), pixel_latents=i["pixel_latents"], plucker=i["plucker"],
-        skeletons=i["skeletons"], cond_mask=i["cond_mask"], timestep_indices=i["timestep_indices"], domain="spatial",
+        skeletons=i["skeletons"].float(), cond_mask=i["cond_mask"], timestep_indices=i["timestep_indices"], domain="spatial",
         guidance_scale=c["guidance"], num_inference_steps=2, enable_pose_encoder=c["pose"])
     torch.testing.assert_close(lat, c["out_latents"], rtol=1e-5, atol=1e-6)
     assert torch.equal(ti, c["out_timestep_indices"])
@@ -189,8 +190,8 @@ def test_sliding_loop_matches_reference_pipeline_golden(tag):
             assert torch.equal(got, ref)
     s = DDIMOracle(SchedulerConfig())
     out = sliding_iterative_denoise_oracle(
-        _fake_unet(11), s, pixel_latents=i["pixel_latents"], plucker=i["plucker"], skeletons=i["skeletons"], cond_mask=mask,
-        latents=i["latents"], domain=c["domain"], timestep_indices=i["timestep_indices"], window_size=c["window_size"],
+        _fake_unet(11), s, pixel_latents=i["pixel_latents"], plucker=i["plucker"], skeletons=i["skeletons"].float(),
+        cond_mask=mask, latents=i["latents"], domain=c["domain"], timestep_indices=i["timestep_indices"], window_size=c["window_size"],
         sliding_stride=c["sliding_stride"], bidirectional=c["bidirectional"], num_denoising_steps=1,
         alternation_rounds=c["alternation_rounds"], guidance_scale=2.0, enable_pose_encoder=True)
     torch.testing.assert_close(out["latents"], c["out_latents"], rtol=1e-5, atol=1e-6)
